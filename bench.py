@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's own CPU path (oracle/_ref)
+    python bench.py ... --dump-outputs DIR     # + what the last timed step computed, as DIR/<name>.npy
 
 One JSON line on rank 0.  Workloads (BASELINE.json configs, synthetic, generated in HBM; every file is far
 larger than L2, so no flush is needed between steps):
@@ -22,6 +23,8 @@ larger than L2, so no flush is needed between steps):
   "bgzf" (C5)     N = 1: the C2 file as BGZF (zlib level 6): member walk + GPU inflate + scan + 1M fetches.
   "e2e"           the call a user makes: pyfastx_b200.Fasta(path) on a tmpfs file -- staging (pread -> pinned ->
                   H2D), scan, names D2H, `.fxi` written by the native bulk writer.
+Every arm times --steps K steps: the scans and extractions after --warmup W (at least 3) steps, the e2e and BGZF
+builds after one warm-up build (e2e: median, BGZF: best of the K builds).
 Parity (rank-local, before anything is reported): ALL rows of C2 and C4 against the CPU oracle (oracle/fxo.c)
 on the downloaded range, >= 3M C4 reads and a C2 sample against the compiled reference (oracle/_ref), ALL 10M
 C3 outputs byte-compared with the oracle, C5 inflated bytes == input bytes.
@@ -41,15 +44,64 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                      # the tree may be read-only: no __pycache__ written into it
 
 SEED_FASTA = 20240601
 SEED_FASTQ = 20240602
 SEED_QUERIES = 123
+SEED_DUMP = 7
 FQ_FIXED = 5 + 11 + 1 + 150 + 1 + 2 + 150 + 1      # "@read" + " 1:N:0:ACGT" + "\n" + seq "\n" "+\n" qual "\n"
+DUMP_ROW_BLOCKS, DUMP_QUERIES, DUMP_LIMIT = 128, 1024, 64 << 20
 
 
 def log(*a):
     print("[bench]", *a, file=sys.stderr, flush=True)
+
+
+# ---------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed step computed (rank 0), for comparing two builds output for output.  Outputs
+# too large to keep whole are sampled at indices fixed by SEED_DUMP; 64 MB in all.
+# ---------------------------------------------------------------------------------------------
+def dump(c, name, a, dtype=np.float64):
+    a = np.ascontiguousarray(a, dtype=dtype)
+    c.dump_bytes += a.nbytes
+    assert c.dump_bytes <= DUMP_LIMIT, "--dump-outputs: more than %d bytes" % DUMP_LIMIT
+    np.save(os.path.join(c.dump, name + ".npy"), a)
+
+
+def dump_sample(n, count):
+    """sorted indices of a fixed sample of `count` of n items (all of them when n <= count)"""
+    if n <= count:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(SEED_DUMP).choice(n, size=count, replace=False))
+
+
+def dump_rows(c, name, d_rows, st, dtype):
+    """scan stats and DUMP_ROW_BLOCKS blocks of 1024 consecutive rows from the device: <name>_row (the row numbers),
+    <name>_<field> per field"""
+    n_rows, blk = int(st["n_rows"]), 1024
+    parts = []
+    for a in dump_sample(-(-n_rows // blk), DUMP_ROW_BLOCKS) * blk:
+        part = np.zeros(min(blk, n_rows - a), dtype=dtype)
+        c.check(c.L.fxg_rows_download(c.eng.ctx, d_rows + int(a) * dtype.itemsize, part.size, dtype.itemsize, part.ctypes.data))
+        parts.append((np.arange(a, a + part.size), part))
+    rows = np.concatenate([p for _, p in parts]) if parts else np.zeros(0, dtype=dtype)
+    dump(c, name + "_stats", [st[k] for k in ("n_rows", "n_lines", "total_len", "end_position", "lead_lines", "lead_bytes", "lead_llen")])
+    dump(c, name + "_row", np.concatenate([i for i, _ in parts]) if parts else [])
+    for f in dtype.names:
+        if f != "pad":
+            dump(c, name + "_" + f, rows[f])
+
+
+def dump_extract(c, label, d_off, d_out):
+    """a fixed sample of DUMP_QUERIES queries of an extraction: extract_<label>_query (query numbers), _length, _bytes"""
+    off = d_off.cpu().numpy()
+    sel = dump_sample(off.size - 1, DUMP_QUERIES)
+    pos = np.concatenate([np.arange(off[i], off[i + 1]) for i in sel])
+    out = d_out[c.torch.from_numpy(pos).to(d_out.device)].cpu().numpy()
+    dump(c, "extract_%s_query" % label, sel)
+    dump(c, "extract_%s_length" % label, off[sel + 1] - off[sel])
+    dump(c, "extract_%s_bytes" % label, out, np.float32)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -438,6 +490,10 @@ def setup(args):
     c.peak, c.peak_src = measured_peaks()
     c.check = _cabi.check
     _cabi.check(c.L.fxg_profile_enable(c.eng.ctx, 1))
+    c.dump = args.dump_outputs if c.rank == 0 else None
+    c.dump_bytes = 0
+    if c.dump:
+        os.makedirs(c.dump, exist_ok=True)
     return c
 
 
@@ -549,16 +605,20 @@ def run_fasta(c, args, result):
     clocks = ClockSampler(c.local)
     clocks.start()
     t = timed_scan(c, dfile, 0, q0, args.steps, args.warmup)
-    # keep the GPU busy for >= 1 s in total so that nvidia-smi sees the load (clock / throttle record)
-    busy_t0 = time.perf_counter()
-    while time.perf_counter() - busy_t0 < 1.2:
+    from pyfastx_b200 import engine
+    if c.dump:
+        dump_rows(c, "fasta_rows", t["d_rows"], t["st"], engine.FASTA_ROW)
+    if args.dump_outputs:
+        barrier(c)                                      # rank 0 dumped alone; the scans below are collective
+    # keep the GPU busy for >= 1 s in total so that nvidia-smi sees the load (clock / throttle record).  Every scan is a
+    # collective exchange, so every rank runs the same number of them, from the step time all ranks agree on.
+    for _ in range(int(1200.0 * args.steps / t["elapsed_ms"]) + 1):
         eng.scan_sharded_dev(c.comm.handle, dfile, 0, q0)
     barrier(c)
     clk = clocks.stop()
     total_bytes = allsum(c, shard_bytes)
     st, infos = t["st"], t["infos"]
     n_rows = st["n_rows"]
-    from pyfastx_b200 import engine
     rows = np.zeros(n_rows, dtype=engine.FASTA_ROW)
     c.check(L.fxg_rows_download(eng.ctx, t["d_rows"], n_rows, 48, rows.ctypes.data))
     assert n_rows == info["records"][1] - info["records"][0], "row count differs from the generator's"
@@ -628,6 +688,8 @@ def run_extract(c, args, dfile, info, rows, result, host_file):
             x1.record(c.stream)
             barrier(c)
             launches = L.fxg_ctx_launch_count(eng.ctx) - l0
+            if c.dump:
+                dump_extract(c, label, d_ooff, d_out)
         x_ms = allmax(c, x0.elapsed_time(x1))
         tot_bases = allsum(c, bases)
         g_ms = float(np.mean(gms))
@@ -647,7 +709,6 @@ def run_extract(c, args, dfile, info, rows, result, host_file):
         out["config"] = {"workload": "C3: %d random (record, start, end, strand) queries per GPU on its resident range, 1 kb "
                                      "windows, strand '-' (reverse-complement) with p=0.5; mixed_length = L ~ U[50, 5000]" % nq}
         # ---- e2e: host queries -> packed bytes on the host, through the C-ABI ----
-        e2e_steps = max(1, min(args.steps, args.e2e_steps))
         out_host, hp2 = pinned_array(bases + 64, np.uint8)
         q_pinned = []
         for arr in (rid, qs, qe):
@@ -663,12 +724,12 @@ def run_extract(c, args, dfile, info, rows, result, host_file):
         e2e_extract()
         barrier(c)
         t0 = time.perf_counter()
-        for _ in range(e2e_steps):
+        for _ in range(args.steps):
             e2e_extract()
         torch.cuda.synchronize()
         e2e_x = allmax(c, time.perf_counter() - t0)
-        out["e2e"] = {"value": tot_bases * e2e_steps / e2e_x / 1e6, "unit": "Mbases/s",
-                      "h2d_bytes_per_step": nq * 28, "d2h_bytes_per_step": bases + (nq + 1) * 8, "steps": e2e_steps,
+        out["e2e"] = {"value": tot_bases * args.steps / e2e_x / 1e6, "unit": "Mbases/s",
+                      "h2d_bytes_per_step": nq * 28, "d2h_bytes_per_step": bases + (nq + 1) * 8, "steps": args.steps,
                       "api": "fxg_extract_host (pinned host queries -> packed bytes on host)"}
         # ---- parity: ALL queries, byte for byte, against oracle/fxo.c on the downloaded range ----
         if host_file is not None and not args.no_parity:
@@ -698,9 +759,8 @@ def run_e2e_and_cpu(c, args, info, rows, st, host_file, result):
     pyfastx_ref = load_reference()
     try:
         # ---- the drop-in call: Fasta(path) = stage + scan + names + .fxi write ----
-        e2e_steps = max(1, min(args.steps, args.e2e_steps))
         times, parts = [], None
-        for k in range(e2e_steps + 1):                       # first build is the warm-up
+        for k in range(args.steps + 1):                       # first build is the warm-up
             if os.path.exists(path + ".fxi"):
                 os.unlink(path + ".fxi")
             t0 = time.perf_counter()
@@ -708,7 +768,7 @@ def run_e2e_and_cpu(c, args, info, rows, st, host_file, result):
             dt = time.perf_counter() - t0
             if k:
                 times.append(dt)
-            if k == e2e_steps:
+            if k == args.steps:
                 assert len(fa) == n_rows and fa.size == int(st["total_len"])
                 assert np.array_equal(fa._rows["boff"], rows["boff"] - info["range"][0])
                 # the reference's per-object idiom through this package (a GPU round trip per query)
@@ -747,7 +807,7 @@ def run_e2e_and_cpu(c, args, info, rows, st, host_file, result):
             del fa
         best = float(np.median(times))                          # median of the measured builds (the first one is the warm-up)
         result["e2e"] = {"value": shard_bytes / best / 1e9, "unit": "GB/s", "h2d_bytes_per_step": int(shard_bytes),
-                         "d2h_bytes_per_step": int(n_rows * 48 + int(rows["nlen"].sum())), "steps": e2e_steps,
+                         "d2h_bytes_per_step": int(n_rows * 48 + int(rows["nlen"].sum())), "steps": args.steps,
                          "seconds_per_build": best,
                          "api": "pyfastx_b200.Fasta(path): tmpfs file -> pinned chunks -> HBM -> scan -> rows + names on host "
                                 "-> .fxi written (native bulk writer, %d B)" % fxi_bytes}
@@ -836,10 +896,9 @@ def run_e2e_sharded(c, args, dfile, info, rows, st, host_file, result):
     if c.rank == 0:
         log("wrote %s (%.2f GB, %d ranks in parallel) in %.1f s" % (path, S / 1e9, c.world, time.perf_counter() - t0))
     try:
-        e2e_steps = max(1, min(args.steps, args.e2e_steps))
         times = []
         res = None
-        for k in range(e2e_steps + 1):                       # first build is the warm-up
+        for k in range(args.steps + 1):                       # first build is the warm-up
             if c.rank == 0 and os.path.exists(path + ".fxi"):
                 os.unlink(path + ".fxi")
             barrier(c)
@@ -858,7 +917,7 @@ def run_e2e_sharded(c, args, dfile, info, rows, st, host_file, result):
         best = float(np.median(times))                          # median of the measured builds (the first one is the warm-up)
         if c.rank == 0:
             result["e2e"] = {"value": S / best / 1e9, "unit": "GB/s", "h2d_bytes_per_step": int(S),
-                             "d2h_bytes_per_step": int(int(args.records) * c.world * 48 + names_bytes), "steps": e2e_steps,
+                             "d2h_bytes_per_step": int(int(args.records) * c.world * 48 + names_bytes), "steps": args.steps,
                              "seconds_per_build": best,
                              "api": "pyfastx_b200.shard.build_index_sharded(path, 'fasta') on %d ranks: ONE tmpfs file of %.2f GB -> every rank "
                                     "stages its byte range (pread -> pinned ring -> HBM) -> sharded scan -> rows + names gathered to rank 0 "
@@ -930,6 +989,8 @@ def run_fastq(c, args, result):
     shard_bytes = q1 - q0
     log("rank %d: FASTQ range [%d, %d) of %d (nominal [%d, %d)), %.3f GB" % (c.rank, q0, q1, S, p0, p1, shard_bytes / 1e9))
     t = timed_scan(c, dfile, 1, q0, args.steps, args.warmup)
+    if c.dump:
+        dump_rows(c, "fastq_rows", t["d_rows"], t["st"], engine.FASTQ_ROW)
     st, infos = t["st"], t["infos"]
     n_rows = st["n_rows"]
     total_reads = allsum(c, n_rows)
@@ -1050,7 +1111,7 @@ def run_bgzf(c, args, dfile_plain, rows_plain, drows, host_file, result):
     zpin[:] = z
     del z
     best, f = None, None
-    for k in range(3):
+    for k in range(args.steps + 1):                         # first build is the warm-up
         if f is not None:
             f.free()
         t0 = time.perf_counter()
@@ -1067,7 +1128,7 @@ def run_bgzf(c, args, dfile_plain, rows_plain, drows, host_file, result):
         t_scan = time.perf_counter() - t2
         recd = {"walk_s": t_walk, "stage_plus_inflate_s": t_inf, "inflate_kernel_ms": inflate_ms, "scan_s": t_scan,
                 "total_s": time.perf_counter() - t0}
-        if best is None or recd["total_s"] < best["total_s"]:
+        if k and (best is None or recd["total_s"] < best["total_s"]):
             best = recd
     assert tot.value == total and f.size == total
     # parity: inflated bytes == the input bytes; rows == the plain-file rows; fetches == the plain-file fetches
@@ -1092,7 +1153,7 @@ def run_bgzf(c, args, dfile_plain, rows_plain, drows, host_file, result):
                                    total / 1e9, args.bgzf_level, nm.value, zpin.size / 1e9)},
         "members": nm.value, "compressed_gb": zpin.size / 1e9, "uncompressed_gb": total / 1e9,
         "inflate_kernel_ms": best["inflate_kernel_ms"], "inflate_GBps_output": total / (best["inflate_kernel_ms"] * 1e-3) / 1e9,
-        "timing_s": best, "host_compress_s": t_comp,
+        "timing_s": best, "steps": args.steps, "host_compress_s": t_comp,
         "fetch": {"queries": nq, "seconds_host_to_host": t_fetch, "Mbases_per_s": float((e - s).sum()) / t_fetch / 1e6},
         "parity": {"inflated_bytes_equal_input": int(total), "rows_equal_plain_scan": int(len(rows)),
                    "fetches_compared_with_oracle": int(n_cmp)}}
@@ -1173,7 +1234,6 @@ def main():
     ap.add_argument("--fastq-reads", type=float, default=126e6, help="C4: reads of the ONE FASTQ file (126M = 41.5 GB)")
     ap.add_argument("--bgzf-queries", type=float, default=1e6)
     ap.add_argument("--bgzf-level", type=int, default=6)
-    ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--ref-sample-records", type=float, default=50000,
                     help="bounded CPU sample for cpu_baseline: 50k records = 0.51 GB")
     ap.add_argument("--ref-fastq-reads", type=float, default=3e6, help="C4 reads checked against the compiled reference")
@@ -1183,7 +1243,11 @@ def main():
     ap.add_argument("--skip-fastq", action="store_true")
     ap.add_argument("--skip-bgzf", action="store_true")
     ap.add_argument("--skip-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (fixed samples of large outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs: the b200 arm only")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":

@@ -4,7 +4,6 @@ test_fastq.py, test_read.py) with the golden vectors standing in for pyfaidx."""
 import gzip
 import os
 import sqlite3
-import sys
 
 import numpy as np
 import pytest
@@ -13,7 +12,6 @@ import goldenlib as G
 import pyfastx_b200 as pyfastx
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def fxi_rows(path, table):
@@ -172,42 +170,33 @@ def test_fastq_api_golden(tmp_path, case):
         fq["definitely-not-a-read"]
 
 
-def _ref():
-    d = os.path.join(ROOT, "oracle", "_ref")
-    if not os.path.isdir(d):
-        return None
-    if d not in sys.path:
-        sys.path.insert(0, d)
-    try:
-        import pyfastx as ref
-        return ref
-    except Exception:
-        return None
-
-
 def test_fxi_interoperates_with_reference(tmp_path):
-    """the reference loads an index written here, and we load one written by the reference"""
-    ref = _ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not available")
+    """the reference loads an index written here, and we load one written by the reference: an index written here
+    has the digest of the file the reference loaded as its own (tests/golden/make_golden_interop.py), whose records
+    it served as recorded there; the reference-written index is stored under tests/golden/data"""
     data = gzip.open(os.path.join(G.GOLD, "data", "test.fa.gz")).read()
     ours = write(tmp_path, "ours.fa", data)
     fa = pyfastx.Fasta(ours)                       # writes ours.fa.fxi on the GPU path
-    rf = ref.Fasta(ours)                           # reference loads OUR index (does not rebuild)
-    assert len(rf) == len(fa) == 211
-    for i in (0, 17, 210):
-        assert rf[i].seq == fa[i].seq and rf[i].name == fa[i].name
-        assert rf[i][5:50].antisense == fa[i][5:50].antisense
+    gold = G.interop("fxi_test_fa")
+    assert G.fxi_digest(ours + ".fxi") == gold["digest"]
+    assert gold["len"] == len(fa) == 211
+    for i, name, n, seq, anti in gold["records"]:
+        assert G.digest(fa[i].seq) == seq and fa[i].name == name and len(fa[i]) == n
+        assert G.digest(fa[i][5:50].antisense) == anti
     theirs = write(tmp_path, "theirs.fa", data)
-    rf2 = ref.Fasta(theirs)                        # reference builds the index
+    G.reference_index("test.fa", theirs + ".fxi")  # the index the reference built for test.fa
     fb = pyfastx.Fasta(theirs)                     # we load THEIR index
-    assert fb.keys() == [s.name for s in rf2]
-    assert fb[3][10:200].seq == rf2[3][10:200].seq
+    gold = G.interop("ref_test_fa")
+    assert fb.keys() == gold["keys"]
+    assert G.digest(fb[3][10:200].seq) == gold["seq3_10_200"]
     fq_data = gzip.open(os.path.join(G.GOLD, "data", "test.fq.gz")).read()
     oq = write(tmp_path, "ours.fq", fq_data)
     fq = pyfastx.Fastq(oq)
-    rq = ref.Fastq(oq)
-    assert len(rq) == len(fq) == 800 and rq[5].seq == fq[5].seq and rq[799].qual == fq[799].qual
+    gold = G.interop("fxi_test_fq")
+    assert G.fxi_digest(oq + ".fxi") == gold["digest"]
+    assert gold["len"] == len(fq) == 800
+    for i, name, seq, qual in gold["reads"]:
+        assert fq[i].name == name and G.digest(fq[i].seq) == seq and G.digest(fq[i].qual) == qual
 
 
 def test_compiled_object_layer_keys_and_fastx(tmp_path):

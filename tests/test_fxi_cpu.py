@@ -1,36 +1,18 @@
 """Host logic of the .fxi writer / loader (pyfastx_b200/fxi.py) without a GPU: rows produced by the CPU
-oracle are written with the reference's schema; the compiled reference (oracle/_ref, when built) must open
-that file as its own index and serve the right sequences, and an index written by the reference must load
-back into the same rows."""
+oracle are written with the reference's schema; the compiled reference opened such files as its own index and
+served the right sequences (tests/golden/make_golden_interop.py recorded those files' digests and its answers),
+and an index written by the reference must load back into the same rows."""
 import gzip
 import os
 import sqlite3
-import sys
 
 import numpy as np
-import pytest
 
 import gen
 import goldenlib as G
 from oracle import fxo
 from pyfastx_b200 import fxi
 from pyfastx_b200._cabi import FASTA_ROW, FASTQ_ROW
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _ref():
-    d = os.path.join(ROOT, "oracle", "_ref")
-    if not os.path.isdir(d):
-        return None
-    sys.path.insert(0, d)
-    try:
-        import pyfastx
-        return pyfastx
-    except Exception:
-        return None
-    finally:
-        sys.path.remove(d)
 
 
 def as_rows(exp, dtype):
@@ -61,17 +43,14 @@ def test_fasta_fxi_roundtrip_and_reference_reads_it(tmp_path):
     for f in ("boff", "blen", "slen", "llen", "elen", "norm", "dlen"):
         assert np.array_equal(back[f], rows[f]), f
     assert back_names.tolist() == [n.decode() for n in names] and tuple(stat[:2]) == (len(rows), total)
-    ref = _ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built: schema and round trip checked only")
-    mtime = os.path.getmtime(str(path) + ".fxi")
-    rf = ref.Fasta(str(path))                          # must LOAD our index, not rebuild it
-    assert os.path.getmtime(str(path) + ".fxi") == mtime
-    assert len(rf) == len(rows) == 211 and rf.size == total
-    for i in (0, 17, 210):
-        s = rf[i]
-        assert s.name == names[i].decode() and len(s) == int(rows["slen"][i])
-        assert s.seq == fxo.subseq(data, exp[i], 0, int(rows["slen"][i])).decode()
+    # the reference loaded this very file as its index (it did not rebuild it) and served these records
+    gold = G.interop("fxi_test_fa")
+    assert G.fxi_digest(str(path) + ".fxi") == gold["digest"]
+    assert gold["len"] == len(rows) == 211 and gold["size"] == total
+    for i, name, n, seq, anti in gold["records"]:
+        assert name == names[i].decode() and n == int(rows["slen"][i])
+        assert G.digest(fxo.subseq(data, exp[i], 0, int(rows["slen"][i]))) == seq
+        assert G.digest(fxo.subseq(data, exp[i], 5, 50, fxo.REVERSE | fxo.COMPLEMENT)) == anti
 
 
 def test_fastq_fxi_roundtrip_and_reference_reads_it(tmp_path):
@@ -88,24 +67,18 @@ def test_fastq_fxi_roundtrip_and_reference_reads_it(tmp_path):
     for f in ("dlen", "rlen", "soff", "qoff"):
         assert np.array_equal(back[f], rows[f]), f
     assert back_names.tolist() == [n.decode("latin-1") for n in names]
-    ref = _ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
-    rq = ref.Fastq(str(path))
-    assert len(rq) == len(rows)
-    for i in (0, 333, len(rows) - 1):
+    gold = G.interop("fxi_random5_fq")                 # the reference loaded this very file and served these reads
+    assert G.fxi_digest(str(path) + ".fxi") == gold["digest"] and gold["len"] == len(rows)
+    for i, name, seq, qual in gold["reads"]:
         es, eq = fxo.read_fetch(data, exp[i])
-        assert rq[i].seq == es.decode() and rq[i].qual == eq.decode() and rq[i].name == names[i].decode("latin-1")
+        assert G.digest(es) == seq and G.digest(eq) == qual and name == names[i].decode("latin-1")
 
 
 def test_reference_written_index_loads_here(tmp_path):
-    ref = _ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
     data = gen.random_fasta(9, n_records=80)
     path = tmp_path / "r.fa"
     path.write_bytes(data)
-    ref.Fasta(str(path))                               # the reference builds r.fa.fxi
+    G.reference_index("random9.fa", str(path) + ".fxi")    # the index the reference built for r.fa
     con, back, back_names, stat = fxi.load_fasta_index(str(path) + ".fxi")
     con.close()
     exp, total, _ = fxo.fasta_scan(data)
@@ -115,9 +88,9 @@ def test_reference_written_index_loads_here(tmp_path):
 
 
 def _dump(path, tables):
+    """digest of every table's rows, integrity check, index names"""
+    out = {t: G.digest(rows) for t, rows in G.fxi_rows(path, tables).items()}
     db = sqlite3.connect(path)
-    db.text_factory = bytes
-    out = {t: db.execute("SELECT * FROM %s ORDER BY rowid" % t).fetchall() for t in tables}
     ok = db.execute("PRAGMA integrity_check").fetchall()
     idx = sorted(r[0] for r in db.execute("SELECT name FROM sqlite_master WHERE type='index'"))
     db.close()
@@ -126,28 +99,24 @@ def _dump(path, tables):
 
 def test_native_writer_is_select_equal_with_the_reference(tmp_path):
     """the file libfxg writes page by page and the file the reference fills with INSERTs answer every SELECT
-    the same (rows of seq / stat / read compared column by column), and sqlite's integrity_check accepts ours"""
-    ref = _ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
+    the same (rows of seq / stat / read compared column by column, through digests of the reference's rows),
+    and sqlite's integrity_check accepts ours"""
     data = gen.random_fasta(31, n_records=3000, crlf_prob=0.2)
-    a, b = tmp_path / "a.fa", tmp_path / "b.fa"
-    a.write_bytes(data); b.write_bytes(data)
-    ref.Fasta(str(a))
+    b = tmp_path / "b.fa"
+    b.write_bytes(data)
     exp, total, _ = fxo.fasta_scan(data)
     fxi.write_fasta_index(str(b) + ".fxi", as_rows(exp, FASTA_ROW), fxo.fasta_names(data, exp), total).close()
-    ra, _, ia = _dump(str(a) + ".fxi", ("seq", "stat", "comp", "gzindex"))
+    gold = G.interop("ref_random31_fa")
     rb, ok, ib = _dump(str(b) + ".fxi", ("seq", "stat", "comp", "gzindex"))
-    assert ok == [(b"ok",)] and ra == rb and ia == ib == [b"chromidx"]
+    assert ok == [("ok",)] and rb == gold["tables"] and ib == gold["indexes"] == ["chromidx"]
     fq = gen.random_fastq(32, n_reads=5000)
-    a, b = tmp_path / "a.fq", tmp_path / "b.fq"
-    a.write_bytes(fq); b.write_bytes(fq)
-    ref.Fastq(str(a))
+    b = tmp_path / "b.fq"
+    b.write_bytes(fq)
     qexp, size, nlines = fxo.fastq_scan(fq)
     fxi.write_fastq_index(str(b) + ".fxi", as_rows(qexp, FASTQ_ROW), fxo.fastq_names(fq, qexp), nlines, size).close()
-    ra, _, ia = _dump(str(a) + ".fxi", ("read", "stat", "base", "meta", "gzindex"))
+    gold = G.interop("ref_random32_fq")
     rb, ok, ib = _dump(str(b) + ".fxi", ("read", "stat", "base", "meta", "gzindex"))
-    assert ok == [(b"ok",)] and ra == rb and ia == ib == [b"readidx"]
+    assert ok == [("ok",)] and rb == gold["tables"] and ib == gold["indexes"] == ["readidx"]
 
 
 def test_native_writer_edge_cases(tmp_path):
@@ -197,10 +166,9 @@ def test_packed_names_table():
 
 
 def test_gz_index_rows_pass_the_reference_import(tmp_path):
-    """a .fxi written for a BGZF input carries zran-layout gzindex rows (src/util.c:442-540): the reference opens it
-    (pyfastx_load_gzip_index, src/util.c:744-767) and serves sequences through it"""
+    """a .fxi written for a BGZF input carries zran-layout gzindex rows (src/util.c:442-540): the reference opened it
+    (pyfastx_load_gzip_index, src/util.c:744-767) and served sequences through it"""
     import struct, zlib
-    ref = _ref()
     data = gen.random_fasta(12, n_records=300, crlf_prob=0.0)
     blocks = []
     for o in range(0, len(data), 0xff00):
@@ -229,10 +197,10 @@ def test_gz_index_rows_pass_the_reference_import(tmp_path):
     assert len(blobs) == 8 + 4 * npts and blobs[0] == b"GZIDX" and blobs[1] == b"\x01"
     assert struct.unpack("<Q", blobs[3])[0] == len(z) and struct.unpack("<Q", blobs[4])[0] == len(data)
     assert struct.unpack("<I", blobs[5])[0] >= struct.unpack("<I", blobs[6])[0] >= 32768
-    if ref is None:
-        pytest.skip("oracle/_ref not built: row layout checked only")
-    mtime = os.path.getmtime(str(path) + ".fxi")
-    rf = ref.Fasta(str(path))
-    assert os.path.getmtime(str(path) + ".fxi") == mtime and len(rf) == len(exp)
-    for i in (0, 150, 299):
-        assert rf[i].seq == fxo.subseq(data, exp[i], 0, int(exp["slen"][i])).decode()
+    # the reference imported a file with these tables and these gzindex field widths, and served these records
+    gold = G.interop("fxi_bgzf_random12")
+    assert G.fxi_digest(str(path) + ".fxi", skip=("gzindex",)) == gold["digest"]
+    assert [len(b) for b in blobs] == gold["gzindex"]["header"] + gold["gzindex"]["point"] * npts
+    assert gold["len"] == len(exp)
+    for i, seq in gold["records"]:
+        assert G.digest(fxo.subseq(data, exp[i], 0, int(exp["slen"][i]))) == seq

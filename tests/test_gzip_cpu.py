@@ -1,24 +1,22 @@
 """Generic (non-BGZF) gzip on the host (csrc/fxg_gzip.cpp): the one sequential zlib pass must reproduce the input
 and every checkpoint it collects must be a REAL zran access point -- raw inflate restarted there with
 inflatePrime(bits) + inflateSetDictionary(window) yields exactly the bytes that follow.  The rows the .fxi then
-carries pass the reference's import (src/util.c:575-609) and the reference serves sequences through our index."""
+carries pass the reference's import (src/util.c:575-609) and the reference serves sequences through our index
+(recorded by tests/golden/make_golden_interop.py)."""
 import ctypes as C
 import gzip
-import os
 import sqlite3
 import struct
-import sys
 import zlib
 
 import numpy as np
 import pytest
 
 import gen
+import goldenlib as G
 from oracle import fxo
 from pyfastx_b200 import _cabi, fxi
 from pyfastx_b200._cabi import FASTA_ROW
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def inflate_host(z, spacing=0):
@@ -87,20 +85,6 @@ def test_concatenated_members_and_corrupt_streams():
         inflate_host(gzip.compress(a)[:-20])
 
 
-def _ref():
-    d = os.path.join(ROOT, "oracle", "_ref")
-    if not os.path.isdir(d):
-        return None
-    sys.path.insert(0, d)
-    try:
-        import pyfastx
-        return pyfastx
-    except Exception:
-        return None
-    finally:
-        sys.path.remove(d)
-
-
 def test_fxi_for_plain_gzip_carries_windows_and_the_reference_opens_it(tmp_path):
     raw = gen.random_fasta(21, n_records=900, crlf_prob=0.0)
     z = gzip.compress(raw, compresslevel=6)
@@ -130,10 +114,10 @@ def test_fxi_for_plain_gzip_carries_windows_and_the_reference_opens_it(tmp_path)
     assert np.array_equal(hs, pts["has"]) and wn.tobytes() == pts["win"]
     _cabi.lib().fxg_gzip_free(h)
     assert fxi.read_gzindex(str(tmp_path / "absent.fxi")) is None
-    ref = _ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built: row layout checked only")
-    mtime = os.path.getmtime(str(path) + ".fxi")
-    rf = ref.Fasta(str(path))
-    assert os.path.getmtime(str(path) + ".fxi") == mtime and len(rf) == len(exp)
-    assert rf[len(exp) - 1].seq == fxo.subseq(raw, exp[-1], 0, int(exp["slen"][-1])).decode()
+    # the reference imported a file with these tables and these gzindex field widths, and served this record
+    gold = G.interop("fxi_gzip_random21")
+    assert G.fxi_digest(str(path) + ".fxi", skip=("gzindex",)) == gold["digest"]
+    assert [len(b) for b in blobs[:8 + 4 * k]] == gold["gzindex"]["header"] + gold["gzindex"]["point"] * k
+    assert gold["len"] == len(exp)
+    for i, seq in gold["records"]:
+        assert G.digest(fxo.subseq(raw, exp[i], 0, int(exp["slen"][i]))) == seq
